@@ -62,6 +62,8 @@ def parse_args():
     ap.add_argument("--legs", default="10,21,41", help="levels timed kernel-only next to the headline level ('' = none)")
     ap.add_argument("--mode", default="default", choices=["default", "one-stream"],
                     help="one-stream: run the NCCL scatter/gather form also at N = 1 (it always runs at N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, to compare two builds")
     return ap.parse_args()
 
 
@@ -300,6 +302,26 @@ def load_peaks():
     return hbm_peak, src
 
 
+DUMP_BLOCKS = 32            # blocks of the sample; with their compressed streams about 34 MB of float32
+
+
+def dump_outputs(out_dir, torch, d_comp, d_csize, d_back, d_dsize, stride, n):
+    """Writes what the last timed step handed a caller of LizardB200_compress_device / _decompress_device: every block's
+    compressed and decompressed size, and for a fixed, seeded sample of blocks the compressed stream (zeros behind its
+    size) and the decompressed bytes, byte values as float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    pick = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_BLOCKS), replace=False))
+    idx = torch.from_numpy(pick).to(d_comp.device)
+    csize = d_csize.cpu().numpy()
+    comp = d_comp.view(n, stride).index_select(0, idx).cpu().numpy().astype(np.float32)
+    comp[np.arange(stride)[None, :] >= np.maximum(csize[pick], 0)[:, None]] = 0.0
+    back = d_back.view(n, BS).index_select(0, idx).cpu().numpy().astype(np.float32)
+    for name, a in (("compressed_sizes", csize.astype(np.float64)), ("decompressed_sizes", d_dsize.cpu().numpy().astype(np.float64)),
+                    ("sample_blocks", pick.astype(np.float64)), ("sample_compressed", comp), ("sample_decompressed", back)):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import lizard_b200 as lz
@@ -392,6 +414,8 @@ def run_ours(args, rank, world, local_rank):
     time.sleep(0.3)
     # ---- headline: timed region of exactly K steps, CUDA events on the launching stream, barrier + sync on both sides ----
     t_c, t_d, comp_total, launches = codec_leg(level, K, W, True)
+    if args.dump_outputs and rank == 0:                 # before the other levels reuse the buffers
+        dump_outputs(args.dump_outputs, torch, d_comp, d_csize, d_back, d_dsize, stride, n)
 
     # ---- the other BASELINE levels, kernel-only, same buffers (configs[2] level -21, configs[3] level -41) ----
     leg_levels = [int(x) for x in args.legs.split(",") if x.strip()] if args.legs else []

@@ -1,12 +1,14 @@
-"""Generate tests/golden/golden.json from the UNMODIFIED reference compiled at oracle/_ref
-(`make -C oracle ref`, sources read in place from /root/reference, -DLIZARD_RESET_MEM build).
-Run in the build container only:  python tests/golden/make_golden.py
-The fixtures let the GPU box (where /root/reference does not exist) and later rounds check the oracle
-and the CUDA path against reference outputs without the reference being present."""
+"""Generate tests/golden/golden.json and tests/golden/optimal_parser_streams.npz from the UNMODIFIED reference compiled
+at oracle/_ref (`make -C oracle ref REF=<reference checkout>`, -DLIZARD_RESET_MEM build):
+    python tests/golden/make_golden.py
+The fixtures let any machine check the oracle and the CUDA path against reference outputs without the reference
+being present.  The recorded answers of tests/golden/reference_calls.bin are made by the suite itself (tests/refs.py)."""
 import hashlib
 import json
 import os
 import sys
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
@@ -63,3 +65,13 @@ for name, data in small:
 with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden.json"), "w") as f:
     json.dump(out, f, indent=0)
 print("wrote golden.json:", len(out["compress"]), "compress facts,", len(out["vectors"]), "vectors")
+
+# streams of the lowest-price (24) and optimal (45) parsers, which the oracle does not restate: decoder inputs for
+# test_*::*stored_optimal_parser_streams, named L<level>_n<size>_p<match pct>_s<seed> after their datagen input
+streams = {}
+for level in (24, 45):
+    for size, pct, seed in ((BS, 90, 1), (BS + 3000, 90, 3), (40000, 50, 4)):
+        c = refs.ref_compress(ref, lz.datagen(size, pct, seed), level)
+        streams["L%d_n%d_p%d_s%d" % (level, size, pct, seed)] = np.frombuffer(c, dtype=np.uint8)
+np.savez_compressed(os.path.join(os.path.dirname(os.path.abspath(__file__)), "optimal_parser_streams.npz"), **streams)
+print("wrote optimal_parser_streams.npz:", sum(len(v) for v in streams.values()), "bytes of streams")

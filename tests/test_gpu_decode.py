@@ -14,10 +14,7 @@ DEFAULT_VARIANT = 7          # the library's default (api.cu Context::dec_varian
 
 @pytest.fixture(scope="module")
 def ref():
-    L = refs.ref_parity()
-    if L is None:
-        pytest.skip("oracle/_ref not built")
-    return L
+    return refs.reference()
 
 
 @pytest.fixture(scope="module")
@@ -36,11 +33,11 @@ def decode_generation(request):
     L.LizardB200_setDecodeVariant(DEFAULT_VARIANT)
 
 
-@pytest.mark.parametrize("level", [10, 21, 41, 30, 11, 17, 24, 45])
+@pytest.mark.parametrize("level", [10, 21, 41, 30, 11, 17, 22, 42])
 def test_decode_blocks_match_original(ref, data4m, level):
     n = 32 if level in (10, 21, 41) else 6
     blocks = [data4m[i * BS:(i + 1) * BS] for i in range(n)]
-    comp = [refs.ref_compress(ref, b, level) for b in blocks]
+    comp = [ref.compress(b, level) for b in blocks]
     out = lz.decompress_batch(comp, [BS] * len(comp))
     for i, (r, o) in enumerate(out):
         assert r == BS, (level, i, r)
@@ -50,7 +47,7 @@ def test_decode_blocks_match_original(ref, data4m, level):
 @pytest.mark.parametrize("level", [10, 21, 41])
 def test_decode_multi_inner_block_unit(ref, data4m, level):
     data = data4m[: 5 * BS + 12345]
-    comp = refs.ref_compress(ref, data, level)
+    comp = ref.compress(data, level)
     r, o = lz.decompress(comp, len(data))
     assert r == len(data) and o == data
 
@@ -60,14 +57,14 @@ def test_decode_edge_sizes(ref):
     cases = [b"", b"a", b"ab" * 10, bytes(100), bytes(BS), bytes(rnd.randrange(256) for _ in range(5000)),
              lz.datagen(1000), lz.datagen(BS + 1), lz.datagen(70000, 90.0, 3)]
     for level in (10, 21, 41):
-        comp = [refs.ref_compress(ref, c, level) for c in cases]
+        comp = [ref.compress(c, level) for c in cases]
         out = lz.decompress_batch(comp, [len(c) for c in cases])
         for c, (r, o) in zip(cases, out):
             assert r == len(c) and o == c, (level, len(c), r)
         # one byte short must fail exactly like the reference (fuzzer property, tests/fuzzer.c:400-404)
         out = lz.decompress_batch(comp, [max(len(c) - 1, 0) for c in cases])
         for c, k, (r, o) in zip(cases, comp, out):
-            rr, _ = refs.ref_decompress(ref, k, max(len(c) - 1, 0))
+            rr, _ = ref.decompress(k, max(len(c) - 1, 0))
             assert r == rr, (level, len(c), r, rr)
 
 
@@ -78,27 +75,15 @@ def test_input_one_byte_short_or_long_matches_reference(ref):
     units, caps = [], []
     for level in (10, 21, 41, 30, 17):
         for blk in (lz.datagen(BS, 50, level), lz.datagen(5000, 50, level), lz.datagen(BS + 777, 50, level), b"", b"a" * 100):
-            comp = refs.ref_compress(ref, blk, level)
+            comp = ref.compress(blk, level)
             for c in (comp[:-1], comp + b"\x00", comp + b"\x80", comp + b"\xff", comp + bytes([rnd.randrange(256)]),
                       comp + bytes(4)):
                 for cap in (len(blk), len(blk) + 64):
                     units.append(c); caps.append(cap)
     got = lz.decompress_batch(units, caps)
     for i, ((r, _), u, cap) in enumerate(zip(got, units, caps)):
-        rr, _ = refs.ref_decompress(ref, u, cap)
+        rr, _ = ref.decompress(u, cap)
         assert r == rr, (i, len(u), cap, r, rr)
-
-
-def _content_is_defined(ref, comp, cap):
-    # The reference copies matches in 8-byte granules, so for offsets < 8 (never produced by any Lizard
-    # encoder) its output depends on stale bytes of dst; only compare contents when decoding into two
-    # differently pre-filled buffers agrees.
-    outs = []
-    for fill in (0x00, 0xA5):
-        dst = ctypes.create_string_buffer(bytes([fill]) * (cap + 64), cap + 64)
-        r = ref.Lizard_decompress_safe(comp, dst, len(comp), cap)
-        outs.append(dst.raw[:max(r, 0)])
-    return outs[0] == outs[1]
 
 
 @pytest.mark.parametrize("level", [10, 21, 41])
@@ -106,7 +91,7 @@ def test_decode_corrupt_matches_reference(ref, data4m, level):
     """Return codes (and bytes when accepted) equal the reference on damaged streams."""
     rnd = random.Random(level)
     blocks = [data4m[i * BS:(i + 1) * BS] for i in range(8)]
-    comp = [refs.ref_compress(ref, b, level) for b in blocks]
+    comp = [ref.compress(b, level) for b in blocks]
     bad, caps = [], []
     for k in comp:
         for _ in range(40):
@@ -127,7 +112,7 @@ def test_decode_corrupt_matches_reference(ref, data4m, level):
     n_cmp = 0
     mism = []
     for idx, (b, cap, (r, o)) in enumerate(zip(bad, caps, out)):
-        rr, ro = refs.ref_decompress(ref, b, cap)
+        rr, ro = ref.decompress(b, cap)
         if r != rr:
             mism.append((idx, len(b), cap, r, rr))
         elif rr > 0 and refs.stream_obeys_min_offset(b, cap):
@@ -138,6 +123,24 @@ def test_decode_corrupt_matches_reference(ref, data4m, level):
     assert n_cmp > 0
 
 
+def test_decode_stored_optimal_parser_streams(ref):
+    """Streams of the reference's lowest-price and optimal parsers (levels 24 and 45; the other tests draw their streams
+    from levels our restatement can compress), valid and damaged, in one batch: same codes and bytes as the reference."""
+    from tests.test_oracle import stored_optimal_parser_cases
+    cases = stored_optimal_parser_cases()
+    got = lz.decompress_batch([c[2] for c in cases], [c[3] for c in cases])
+    compared = 0
+    for (level, data, comp, cap, intact), (r, o) in zip(cases, got):
+        rr, ro = ref.decompress(comp, cap)
+        assert r == rr, (level, len(data), len(comp), cap, r, rr)
+        if intact:
+            assert o == data
+        if rr > 0 and refs.stream_obeys_min_offset(comp, cap):
+            compared += 1
+            assert o == ro, (level, len(data), cap)
+    assert compared > 0
+
+
 def test_decode_schedules_and_prepass_agree(ref, data4m):
     """Every decode configuration (token-loop schedules, with and without the Huffman pre-pass) returns the same
     codes and bytes on a mixed batch: all levels side by side, damaged streams in between, a multi-inner-block unit."""
@@ -146,17 +149,17 @@ def test_decode_schedules_and_prepass_agree(ref, data4m):
     L.LizardB200_setDecodeVariant.argtypes = [ctypes.c_int]
     units, caps = [], []
     for i in range(48):
-        level = [41, 30, 10, 21, 45, 37][i % 6]
+        level = [41, 30, 10, 21, 42, 37][i % 6]
         blk = data4m[i * BS:(i + 1) * BS] if i % 5 else data4m[i * BS:i * BS + rnd.randrange(1, BS)]
-        k = refs.ref_compress(ref, blk, level)
+        k = ref.compress(blk, level)
         units.append(k); caps.append(len(blk))
         b = bytearray(k)
         for _ in range(rnd.randrange(1, 4)):
             b[rnd.randrange(len(b))] ^= 1 << rnd.randrange(8)
         units.append(bytes(b)); caps.append(len(blk))
     big = data4m[: 3 * BS + 555]
-    units.append(refs.ref_compress(ref, big, 41)); caps.append(len(big))
-    want = [refs.ref_decompress(ref, u, c) for u, c in zip(units, caps)]
+    units.append(ref.compress(big, 41)); caps.append(len(big))
+    want = [ref.decompress(u, c) for u, c in zip(units, caps)]
     try:
         for variant in (15, 7, 11, 3, 12, 0, 5, 6, 23, 19, 16):
             assert L.LizardB200_setDecodeVariant(variant) == 0
@@ -181,7 +184,7 @@ def test_device_api_unaligned_destinations(ref, data4m):
         for i in range(24):
             n = BS if i % 3 else rnd.randrange(1, BS)
             blocks.append(data4m[i * BS:i * BS + n])
-            comp.append(refs.ref_compress(ref, blocks[-1], level))
+            comp.append(ref.compress(blocks[-1], level))
         src_off, dst_off, pos_s, pos_d = [], [], 0, 0
         for b, c in zip(blocks, comp):
             pos_s += rnd.randrange(0, 9)

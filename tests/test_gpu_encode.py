@@ -15,10 +15,7 @@ LEVELS = [10, 11, 13, 15, 17, 20, 21, 22, 30, 31, 34, 38, 40, 41, 42]
 
 @pytest.fixture(scope="module")
 def ref():
-    L = refs.ref_parity()
-    if L is None:
-        pytest.skip("oracle/_ref not built")
-    return L
+    return refs.reference()
 
 
 @pytest.fixture(scope="module")
@@ -31,7 +28,7 @@ def test_blocks_bit_exact(ref, data4m, level):
     blocks = [data4m[i * BS:(i + 1) * BS] for i in range(32)]
     out = lz.compress_batch(blocks, level, [BS - 1] * 32)      # frame layer's capacity (lizard_frame.c:459)
     for i, (r, o) in enumerate(out):
-        want = refs.ref_compress(ref, blocks[i], level, BS - 1)
+        want = ref.compress(blocks[i], level, BS - 1)
         assert r == len(want) and o == want, (level, i, r, len(want))
 
 
@@ -39,7 +36,7 @@ def test_blocks_bit_exact(ref, data4m, level):
 def test_multi_inner_block_call_bit_exact(ref, data4m, level):
     """Config 1 of BASELINE.json: one Lizard_compress call over 4 MiB = 32 dependent inner blocks."""
     got = lz.compress(data4m, level)
-    want = refs.ref_compress(ref, data4m, level)
+    want = ref.compress(data4m, level)
     assert got == want
     r, back = lz.decompress(got, len(data4m))
     assert r == len(data4m) and back == data4m
@@ -68,7 +65,7 @@ def test_edge_inputs_and_capacities(ref, level):
         caps.append(rnd.choice([bound, bound, max(len(c) - 1, 1), len(c) // 2 + 1, rnd.randrange(1, bound + 1)]))
     out = lz.compress_batch(cases, level, caps)
     for c, cap, (r, o) in zip(cases, caps, out):
-        want = refs.ref_compress(ref, c, level, cap)
+        want = ref.compress(c, level, cap)
         assert r == len(want) and o == want, (level, len(c), cap, r, len(want))
 
 
@@ -78,12 +75,12 @@ def test_compress_into_exact_and_short_capacity(ref, level):
     gives what the reference gives (0)."""
     units, caps = [], []
     for blk in (lz.datagen(BS, 50, level), lz.datagen(70000, 30, level + 1), lz.datagen(3000, 50, 7), bytes(5000)):
-        full = refs.ref_compress(ref, blk, level)
+        full = ref.compress(blk, level)
         for cap in (len(full), len(full) - 1, len(full) // 2):
             units.append(blk); caps.append(cap)
     out = lz.compress_batch(units, level, caps)
     for blk, cap, (r, o) in zip(units, caps, out):
-        want = refs.ref_compress(ref, blk, level, cap)
+        want = ref.compress(blk, level, cap)
         assert r == len(want) and o == want, (level, len(blk), cap, r, len(want))
 
 

@@ -1,9 +1,9 @@
 """GPU parity at BASELINE.json's full size (configs 1-3: 1 GiB `datagen -P50`, 8192 independent 128 KiB blocks).
 
-The compiled reference needs minutes for 1 GiB per level, so the check goes through the reference-generated facts of
-SURVEY.md section 8c instead -- a checksum of checksums: the input's md5, the total compressed size and the XXH64
-(seed 0, the reference's own lib/xxhash) of the 8192 compressed blocks concatenated, all taken from the reference
-built with -DLIZARD_RESET_MEM (`Lizard_compress(block, cap = srcSize-1)` per block) -- plus the round trip."""
+The compiled reference needs minutes for 1 GiB per level, so the check goes through reference-generated facts instead --
+a checksum of checksums: the input's md5, the total compressed size and the SHA-256 of the 8192 compressed blocks
+concatenated, all taken from the reference built with -DLIZARD_RESET_MEM (`Lizard_compress(block, cap = srcSize-1)` per
+block; the sizes and the XXH64 of the same streams are SURVEY.md section 8c's facts) -- plus the round trip."""
 import ctypes
 import hashlib
 
@@ -11,24 +11,15 @@ import numpy as np
 import pytest
 
 import lizard_b200 as lz
-from tests import refs
 
 pytestmark = pytest.mark.gpu
 BS = lz.BLOCK_SIZE
 N = 1 << 30
-# level -> (compressed bytes, XXH64 of the concatenated blocks): SURVEY.md section 8c
-FACTS_1G = {10: (670259129, 0x9420eb931f31b928), 21: (616060194, 0x3a96889958c29131), 41: (385653946, 0x541a42ece9b3ed90)}
+# level -> (compressed bytes, SHA-256 of the concatenated blocks)
+FACTS_1G = {10: (670259129, "ed6159bb08e1509bc0d585195f1d1d6fc589724749c90b358ab8cc589a89f023"),
+            21: (616060194, "e19093ae2fdfc7f595fb3670323b1d7b535fd9d0abf4e058c6146c1ff9cfc8e4"),
+            41: (385653946, "b564134e421d99fd4687da6fa90e29a30fc60e58f5f410b395e25a05c04b4d90")}
 MD5_1G = "b98d56d2653b6ab1b74ebe6c827ec231"
-
-
-@pytest.fixture(scope="module")
-def ref():
-    L = refs.ref_parity()
-    if L is None:
-        pytest.skip("oracle/_ref not built")
-    L.Lizard_XXH64.restype = ctypes.c_ulonglong
-    L.Lizard_XXH64.argtypes = [ctypes.c_void_p, ctypes.c_size_t, ctypes.c_ulonglong]
-    return L
 
 
 @pytest.fixture(scope="module")
@@ -40,7 +31,7 @@ def data1g():
 
 
 @pytest.mark.parametrize("level", [10, 21, 41])
-def test_one_gib_matches_reference_facts(ref, data1g, level):
+def test_one_gib_matches_reference_facts(data1g, level):
     L = lz.lib()
     L.LizardB200_compress_blocks.argtypes = [ctypes.c_void_p, ctypes.c_size_t, ctypes.c_int, ctypes.c_void_p, ctypes.c_size_t,
                                              ctypes.c_int, ctypes.c_void_p, ctypes.c_int]
@@ -52,7 +43,7 @@ def test_one_gib_matches_reference_facts(ref, data1g, level):
     st = L.LizardB200_compress_blocks(data1g.ctypes.data, N, BS, comp.ctypes.data, BS, BS - 1, sizes.ctypes.data, level)
     assert st == 0, L.LizardB200_lastError()
     assert int(sizes.min()) > 0
-    total, xxh = FACTS_1G[level]
+    total, sha = FACTS_1G[level]
     assert int(sizes.sum(dtype=np.int64)) == total
     packed = np.empty(total, dtype=np.uint8)
     at = 0
@@ -60,7 +51,7 @@ def test_one_gib_matches_reference_facts(ref, data1g, level):
         k = int(sizes[i])
         packed[at:at + k] = comp[i * BS:i * BS + k]
         at += k
-    assert ref.Lizard_XXH64(packed.ctypes.data, total, 0) == xxh
+    assert hashlib.sha256(packed).hexdigest() == sha
     del packed
     back = np.zeros(N, dtype=np.uint8)
     res = np.zeros(n, dtype=np.int32)
